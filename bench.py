@@ -443,6 +443,9 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-vae", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the 12B / I2V / torch-baseline secondary lines")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the latents returned by the last timed step to DIR/latents.npy (float32), so that two builds "
+                         "can be compared on the same seeded inputs")
     args = ap.parse_args()
     preset = PRESETS[args.preset]
     if args.impl == "reference":
@@ -553,6 +556,10 @@ def main():
     ms_total, launches, attn_ms, latents, step_i = timed_steps(sampler, latents, embeds, rope, inpaint, args.steps, args.warmup, True,
                                                                clocks=clocks)
     clock_info = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "latents.npy"), latents.float().cpu().numpy())
 
     # ---- end to end through the public API with HOST buffers (H2D inputs + D2H result every step)
     lat_host = torch.empty(latents.shape, dtype=bf16, pin_memory=True).copy_(latents)

@@ -2,14 +2,15 @@
 against the REFERENCE's own pipeline classes, both over the same product modules with the kernels replaced by the torch
 stand-ins of tests/cpu_ops.py: same inputs, same seeded noise -> the same frames.  What differs between the two runs is only the
 host code under test here (prompt plumbing, latent shapes, noise draw, conditioning preparation, schedule indexing, the fused
-CFG + Euler update instead of four tensor ops, the fused output tail)."""
+CFG + Euler update instead of four tensor ops, the fused output tail).  The reference pipelines' frames are stored results
+(tests/refgold.py); on another CPU configuration they are matched within 3e-2 relative, three times the spread that the CPU
+instruction set and thread count alone cause in these bf16 runs (below 1e-2)."""
 import pytest
 import torch
 
 from oracle import dit, ref_pipeline, vae
-from tests import cpu_ops
+from tests import cpu_ops, refgold
 
-pytestmark = pytest.mark.skipif(not ref_pipeline.available(), reason="/root/reference not present")
 bf16 = torch.bfloat16
 CFG = dict(num_attention_heads=2, attention_head_dim=64, in_channels=16, out_channels=16, patch_size=2, num_layers=2,
            time_embed_dim=64, add_norm_text_encoder=True, text_embed_dim=128, text_embed_dim_t5=None,
@@ -63,9 +64,9 @@ def _mask_kw(pe, ne):
                 prompt_embeds_2=pe, prompt_attention_mask_2=ones.clone())
 
 
-def _same(a, b):
-    assert a.shape == b.shape and a.dtype == b.dtype == torch.float32
-    assert torch.equal(a, b), float((a - b).abs().max())
+def _same(got, want):
+    assert got.dtype == torch.float32
+    refgold.assert_equal(got, want, rel=3e-2)
 
 
 def test_t2v_pipeline_equals_the_reference_pipeline(on_cpu):
@@ -74,29 +75,30 @@ def test_t2v_pipeline_equals_the_reference_pipeline(on_cpu):
     g = torch.Generator().manual_seed(1)
     lat = torch.randn(1, 16, LF, H // 8, W // 8, generator=g).to(bf16)
     pe, ne = _embeds(g)
-    want = ref_pipeline.run(ref_pipeline.reference_pipeline(t, v), lat, pe, ne, height=H, width=W, video_length=FRAMES,
-                            num_inference_steps=STEPS)
+    want = refgold.want("native/t2v", lambda: ref_pipeline.run(ref_pipeline.reference_pipeline(t, v), lat, pe, ne, height=H, width=W,
+                                                               video_length=FRAMES, num_inference_steps=STEPS))
     pipe = EasyAnimatePipeline(vae=v, transformer=t)
     out = pipe(video_length=FRAMES, height=H, width=W, num_inference_steps=STEPS, guidance_scale=6.0, latents=lat, **_mask_kw(pe, ne))
     _same(out.frames, want)
     assert pipe.num_timesteps == STEPS and out[0] is out.frames
     # noise drawn by the pipeline itself: the reference's randn_tensor semantics (CPU generator, transformer dtype)
-    want = ref_pipeline.reference_pipeline(t, v)(video_length=FRAMES, height=H, width=W, num_inference_steps=2, guidance_scale=6.0,
-                                                  generator=torch.Generator().manual_seed(5), **_mask_kw(pe, ne)).frames
+    want = refgold.want("native/t2v_generator", lambda: ref_pipeline.reference_pipeline(t, v)(
+        video_length=FRAMES, height=H, width=W, num_inference_steps=2, guidance_scale=6.0, generator=torch.Generator().manual_seed(5),
+        **_mask_kw(pe, ne)).frames)
     got = pipe(video_length=FRAMES, height=H, width=W, num_inference_steps=2, guidance_scale=6.0,
                generator=torch.Generator().manual_seed(5), **_mask_kw(pe, ne), output_type="numpy", return_dict=False)
     assert isinstance(got, __import__("numpy").ndarray)
     _same(torch.from_numpy(got), want)
     # no guidance (guidance_scale <= 1): one forward per step, no negative prompt needed
-    want = ref_pipeline.reference_pipeline(t, v)(video_length=FRAMES, height=H, width=W, num_inference_steps=2, guidance_scale=1.0,
-                                                  latents=lat, **_mask_kw(pe, ne)).frames
+    want = refgold.want("native/t2v_no_guidance", lambda: ref_pipeline.reference_pipeline(t, v)(
+        video_length=FRAMES, height=H, width=W, num_inference_steps=2, guidance_scale=1.0, latents=lat, **_mask_kw(pe, ne)).frames)
     _same(pipe(video_length=FRAMES, height=H, width=W, num_inference_steps=2, guidance_scale=1.0, latents=lat, **_mask_kw(pe, ne)).frames, want)
 
 
 def test_t2v_pipeline_rejects_what_the_reference_rejects(on_cpu):
     from easyanimate_b200 import EasyAnimatePipeline
     t, v = _modules(on_cpu)
-    pipe, ref = EasyAnimatePipeline(vae=v, transformer=t), ref_pipeline.reference_pipeline(t, v)
+    pipe = EasyAnimatePipeline(vae=v, transformer=t)
     g = torch.Generator().manual_seed(2)
     pe, ne = _embeds(g)
     ok = dict(video_length=FRAMES, height=H, width=W, num_inference_steps=2, guidance_scale=6.0)
@@ -107,12 +109,20 @@ def test_t2v_pipeline_rejects_what_the_reference_rejects(on_cpu):
         dict(ok, prompt="a cat", **_mask_kw(pe, ne)),                                          # both prompt and embeds
         dict(ok, **_mask_kw(pe, ne), callback_on_step_end_tensor_inputs=["nope"]),
     ]
-    for kw in bad_calls:
-        with pytest.raises(ValueError) as e_ref:
-            ref(**kw)
+    def reference_errors():
+        ref, errors = ref_pipeline.reference_pipeline(t, v), []
+        for kw in bad_calls:
+            with pytest.raises(ValueError) as e_ref:
+                ref(**kw)
+            errors.append(str(e_ref.value).split(":")[0][:40])
+        return errors
+
+    want = refgold.want("native/t2v_rejects", reference_errors)
+    assert len(want) == len(bad_calls)
+    for kw, e_ref in zip(bad_calls, want):
         with pytest.raises(ValueError) as e_ours:
             pipe(**kw)
-        assert str(e_ours.value).split(":")[0][:40] == str(e_ref.value).split(":")[0][:40]
+        assert str(e_ours.value).split(":")[0][:40] == e_ref
     with pytest.raises(NotImplementedError):
         pipe(**ok, **_mask_kw(pe, ne), guidance_rescale=0.7)
 
@@ -130,10 +140,15 @@ def test_callback_on_step_end_sees_and_replaces_latents(on_cpu):
         return {"latents": kw["latents"] * 0.5} if i == 0 else {}
 
     kw = dict(video_length=FRAMES, height=H, width=W, num_inference_steps=STEPS, guidance_scale=6.0, latents=lat, **_mask_kw(pe, ne))
-    want = ref_pipeline.reference_pipeline(t, v)(callback_on_step_end=cb, **kw).frames
-    ref_seen, seen[:] = list(seen), []
+    def reference_call():
+        frames = ref_pipeline.reference_pipeline(t, v)(callback_on_step_end=cb, **kw).frames
+        return {"frames": frames, "seen": list(seen)}
+
+    want = refgold.want("native/callback", reference_call)
+    seen[:] = []
     got = EasyAnimatePipeline(vae=v, transformer=t)(callback_on_step_end=cb, **kw).frames
-    assert seen == ref_seen and len(seen) == STEPS
+    assert [[i, t_, list(s)] for i, t_, s in seen] == want["seen"] and len(seen) == STEPS
+    want = want["frames"]
     _same(got, want)
 
 
@@ -149,7 +164,8 @@ def test_inpaint_pipeline_equals_the_reference_pipeline(on_cpu, strength):
     pe, ne = _embeds(g)
     kw = dict(video_length=FRAMES, video=video, mask_video=mask, height=H, width=W, num_inference_steps=4, guidance_scale=6.0,
               strength=strength, noise_aug_strength=0.0563, **_mask_kw(pe, ne))
-    want = ref_pipeline.reference_inpaint_pipeline(t, v)(generator=torch.Generator().manual_seed(9), **kw).frames
+    want = refgold.want(f"native/inpaint_{strength}", lambda: ref_pipeline.reference_inpaint_pipeline(t, v)(
+        generator=torch.Generator().manual_seed(9), **kw).frames)
     got = EasyAnimateInpaintPipeline(vae=v, transformer=t)(generator=torch.Generator().manual_seed(9), **kw).frames
     _same(got, want)
 
@@ -164,7 +180,8 @@ def test_inpaint_pipeline_all_masked_is_zero_conditioning(on_cpu):
     pe, ne = _embeds(g)
     kw = dict(video_length=FRAMES, video=video, mask_video=mask, height=H, width=W, num_inference_steps=2, guidance_scale=6.0,
               **_mask_kw(pe, ne))
-    want = ref_pipeline.reference_inpaint_pipeline(t, v)(generator=torch.Generator().manual_seed(10), **kw).frames
+    want = refgold.want("native/inpaint_all_masked", lambda: ref_pipeline.reference_inpaint_pipeline(t, v)(
+        generator=torch.Generator().manual_seed(10), **kw).frames)
     _same(EasyAnimateInpaintPipeline(vae=v, transformer=t)(generator=torch.Generator().manual_seed(10), **kw).frames, want)
 
 
@@ -182,7 +199,7 @@ def test_control_pipeline_equals_the_reference_pipeline(on_cpu, mode):
         kw["ref_image"] = torch.rand(1, 3, 1, H, W, generator=g)
     if mode == "camera":
         kw["control_camera_video"] = torch.randn(1, 16, FRAMES, H, W, generator=g)
-    want = ref_pipeline.reference_control_pipeline(t, v)(**kw).frames
+    want = refgold.want(f"native/control_{mode}", lambda: ref_pipeline.reference_control_pipeline(t, v)(**kw).frames)
     _same(EasyAnimateControlPipeline(vae=v, transformer=t)(**kw).frames, want)
 
 
@@ -234,18 +251,24 @@ def test_prompt_strings_go_through_the_llm_branch_like_the_reference(on_cpu):
     t, v = _modules(on_cpu)
     torch.manual_seed(0)
     tok, enc = _FakeTokenizer(), _FakeTextEncoder(128).to(bf16)
-    ref = ref_pipeline.reference_pipeline(t, v)
-    ref.tokenizer, ref.text_encoder = tok, enc
     lat = torch.randn(1, 16, LF, H // 8, W // 8, generator=torch.Generator().manual_seed(11)).to(bf16)
     kw = dict(prompt="a corgi surfing", negative_prompt="blurry", video_length=FRAMES, height=H, width=W, num_inference_steps=2,
               guidance_scale=6.0, latents=lat)
-    want = ref(**kw).frames
+
+    def reference_call():
+        ref = ref_pipeline.reference_pipeline(t, v)
+        ref.tokenizer, ref.text_encoder = tok, enc
+        frames = ref(**kw).frames
+        return {"frames": frames, "embeds": ref.encode_prompt("a corgi surfing", torch.device("cpu"), bf16, negative_prompt="blurry")}
+
+    want = refgold.want("native/prompt_strings", reference_call)
     got = EasyAnimatePipeline(vae=v, transformer=t, tokenizer=tok, text_encoder=enc)(**kw).frames
-    _same(got, want)
-    e_ref = ref.encode_prompt("a corgi surfing", torch.device("cpu"), bf16, negative_prompt="blurry")
+    _same(got, want["frames"])
     e_ours = EasyAnimatePipeline(vae=v, transformer=t, tokenizer=tok, text_encoder=enc).encode_prompt(
         "a corgi surfing", torch.device("cpu"), bf16, negative_prompt="blurry")
-    assert all(torch.equal(a, b) for a, b in zip(e_ref, e_ours))
+    assert len(e_ours) == len(want["embeds"])
+    for a, b in zip(e_ours, want["embeds"]):
+        refgold.assert_equal(a, b, rel=3e-2)
 
 
 def test_teacache_inside_the_pipeline_call_matches_the_reference_pipeline(on_cpu):
@@ -260,11 +283,16 @@ def test_teacache_inside_the_pipeline_call_matches_the_reference_pipeline(on_cpu
     steps = 8
     kw = dict(video_length=FRAMES, height=H, width=W, num_inference_steps=steps, guidance_scale=6.0, latents=lat, **_mask_kw(pe, ne))
     t.enable_teacache(steps, 0.3, coefficients=coeffs)
-    want = ref_pipeline.reference_pipeline(t, v)(**kw).frames
-    skipped_ref = t.teacache.skipped
-    assert t.teacache.cnt == 0  # wrapped around after `steps` calls: ready for the next video
+    def reference_call():
+        frames = ref_pipeline.reference_pipeline(t, v)(**kw).frames
+        assert t.teacache.cnt == 0  # wrapped around after `steps` calls: ready for the next video
+        return {"frames": frames, "skipped": t.teacache.skipped}
+
+    want = refgold.want("native/teacache", reference_call)
+    skipped_ref, want = want["skipped"], want["frames"]
+    skipped0 = t.teacache.skipped
     got = EasyAnimatePipeline(vae=v, transformer=t)(**kw).frames
-    assert 0 < skipped_ref < steps and t.teacache.skipped == 2 * skipped_ref
+    assert 0 < skipped_ref < steps and t.teacache.skipped - skipped0 == skipped_ref and t.teacache.cnt == 0
     _same(got, want)
 
 
@@ -275,8 +303,9 @@ def test_two_videos_per_prompt(on_cpu):
     pe, ne = _embeds(torch.Generator().manual_seed(31))
     kw = dict(video_length=FRAMES, height=H, width=W, num_inference_steps=2, guidance_scale=6.0, num_images_per_prompt=2,
               **_mask_kw(pe, ne))
-    ref, pipe = ref_pipeline.reference_pipeline(t, v), EasyAnimatePipeline(vae=v, transformer=t)
-    want = ref(generator=torch.Generator().manual_seed(32), **kw).frames
+    pipe = EasyAnimatePipeline(vae=v, transformer=t)
+    want = refgold.want("native/two_videos", lambda: ref_pipeline.reference_pipeline(t, v)(
+        generator=torch.Generator().manual_seed(32), **kw).frames)
     got = pipe(generator=torch.Generator().manual_seed(32), **kw).frames
     assert got.shape == (2, 3, FRAMES, H, W)
     _same(got, want)
@@ -315,7 +344,8 @@ def test_load_pipeline_follows_the_predict_scripts_loading_sequence(on_cpu, tmp_
               **_mask_kw(pe, ne))
     from easyanimate_b200 import FlowMatchEulerDiscreteScheduler
     by_hand = EasyAnimateInpaintPipeline(vae=v, transformer=t, scheduler=FlowMatchEulerDiscreteScheduler(shift=3.0))
-    _same(pipe(generator=torch.Generator().manual_seed(94), **kw).frames, by_hand(generator=torch.Generator().manual_seed(94), **kw).frames)
+    a, b = pipe(generator=torch.Generator().manual_seed(94), **kw).frames, by_hand(generator=torch.Generator().manual_seed(94), **kw).frames
+    assert a.dtype == b.dtype == torch.float32 and torch.equal(a, b), float((a - b).abs().max())
     # a 16-channel checkpoint gives the text-to-video pipeline
     t16, _ = _modules(on_cpu, seeds=(95, 92))
     (tmp_path / "transformer" / "config.json").write_text(json.dumps(dict(t16.config)))
@@ -332,7 +362,8 @@ def test_t2v_edge_shapes(on_cpu, video_length, h, w):
     t, v = _modules(on_cpu)
     pe, ne = _embeds(torch.Generator().manual_seed(41))
     kw = dict(video_length=video_length, height=h, width=w, num_inference_steps=2, guidance_scale=6.0, **_mask_kw(pe, ne))
-    want = ref_pipeline.reference_pipeline(t, v)(generator=torch.Generator().manual_seed(42), **kw).frames
+    want = refgold.want(f"native/edge_{video_length}x{h}x{w}", lambda: ref_pipeline.reference_pipeline(t, v)(
+        generator=torch.Generator().manual_seed(42), **kw).frames)
     got = EasyAnimatePipeline(vae=v, transformer=t)(generator=torch.Generator().manual_seed(42), **kw).frames
     assert got.shape == (1, 3, video_length, h // 16 * 16, w // 16 * 16)
     _same(got, want)
@@ -350,7 +381,8 @@ def test_inpaint_pipeline_with_vae_encoded_mask(on_cpu):
     pe, ne = _embeds(g)
     kw = dict(video_length=FRAMES, video=video, mask_video=mask, height=H, width=W, num_inference_steps=2, guidance_scale=6.0,
               **_mask_kw(pe, ne))
-    want = ref_pipeline.reference_inpaint_pipeline(t, v)(generator=torch.Generator().manual_seed(15), **kw).frames
+    want = refgold.want("native/inpaint_vae_mask", lambda: ref_pipeline.reference_inpaint_pipeline(t, v)(
+        generator=torch.Generator().manual_seed(15), **kw).frames)
     _same(EasyAnimateInpaintPipeline(vae=v, transformer=t)(generator=torch.Generator().manual_seed(15), **kw).frames, want)
 
 
@@ -368,7 +400,8 @@ def test_inpaint_reference_video_noise_with_sampled_strength(on_cpu):
     kw = dict(video_length=FRAMES, video=video, mask_video=mask, height=H, width=W, num_inference_steps=2, guidance_scale=6.0,
               noise_aug_strength=None, **_mask_kw(pe, ne))
     torch.manual_seed(17)
-    want = ref_pipeline.reference_inpaint_pipeline(t, v)(generator=torch.Generator().manual_seed(18), **kw).frames
+    want = refgold.want("native/inpaint_sampled_strength", lambda: ref_pipeline.reference_inpaint_pipeline(t, v)(
+        generator=torch.Generator().manual_seed(18), **kw).frames)
     torch.manual_seed(17)
     got = EasyAnimateInpaintPipeline(vae=v, transformer=t)(generator=torch.Generator().manual_seed(18), **kw).frames
     _same(got, want)

@@ -1,22 +1,23 @@
-"""SURVEY.md section 8b, the boundary's strongest proof available without a GPU: the REFERENCE's own
-`EasyAnimatePipeline.__call__` (easyanimate/pipeline/pipeline_easyanimate.py:769-1148, executed unmodified from
-/root/reference through oracle/ref_pipeline.py) driving
+"""SURVEY.md section 8b, the boundary's strongest proof available without a GPU: the REFERENCE's own pipeline classes
+(easyanimate/pipeline/pipeline_easyanimate.py:769-1148 and its inpaint / control siblings, executed unmodified through
+oracle/ref_pipeline.py where the original project is installed) over the reference's own transformer + VAE, whose frames are
+stored (tests/refgold.py) and
 
-  (1) the reference's own transformer + VAE  -> pins oracle.dit.denoise_loop + oracle.vae decode + the decode_latents tail
-      (what every GPU parity test compares with) against the reference's loop, not against a restatement of it;
-  (2) the PRODUCT modules (easyanimate_b200.EasyAnimateTransformer3DModel / AutoencoderKLMagvit, kernels replaced by the
-      torch stand-ins of tests/cpu_ops.py) plugged into the same unmodified pipeline object -> every attribute, keyword and
-      return convention the reference pipeline touches exists on the product modules and means the same thing.
+  (1) pin oracle.dit.denoise_loop + oracle.vae decode + the decode_latents tail (what every GPU parity test compares with)
+      against the reference's loop, not against a restatement of it;
+  (2) are what the PRODUCT pipelines over the PRODUCT modules (easyanimate_b200.EasyAnimateTransformer3DModel /
+      AutoencoderKLMagvit, kernels replaced by the torch stand-ins of tests/cpu_ops.py) produce from the same call, up to bf16
+      round-off; tests/test_native_pipelines_cpu.py pins the product pipelines to the reference's over the same modules.
 
-Skipped where /root/reference is absent (the GPU box); the GPU-side counterpart is the fixture `pipe_ref_t2v.safetensors`
-minted by (1) (tests/golden/make_golden.py) and compared with in tests/test_pipeline_gpu.py."""
+The GPU-side counterpart is the fixture `pipe_ref_t2v.safetensors` minted by (1) (tests/golden/make_golden.py) and compared with
+in tests/test_pipeline_gpu.py."""
 import pytest
 import torch
 
 from oracle import dit, ref_pipeline, vae
-from tests import cpu_ops
+from tests import refgold
+from tests.test_native_pipelines_cpu import on_cpu  # noqa: F401  (fixture: product modules on the torch stand-ins)
 
-pytestmark = pytest.mark.skipif(not ref_pipeline.available(), reason="/root/reference not present")
 bf16 = torch.bfloat16
 CFG = dict(num_attention_heads=2, attention_head_dim=64, in_channels=16, out_channels=16, patch_size=2, num_layers=2,
            time_embed_dim=64, add_norm_text_encoder=True, text_embed_dim=128, text_embed_dim_t5=None)
@@ -52,41 +53,38 @@ def _oracle_frames(lat, pe, ne, dtype):
 
 def test_reference_pipeline_call_pins_the_oracle_loop_fp32():
     lat, pe, ne = _inputs()
-    rt, rv = _reference_modules(torch.float32)
-    pipe = ref_pipeline.reference_pipeline(rt, rv)
-    frames = ref_pipeline.run(pipe, lat, pe, ne, height=H, width=W, video_length=FRAMES, num_inference_steps=STEPS)
+    frames = refgold.want("ref_pipeline/fp32", lambda: ref_pipeline.run(
+        ref_pipeline.reference_pipeline(*_reference_modules(torch.float32)), lat, pe, ne, height=H, width=W, video_length=FRAMES,
+        num_inference_steps=STEPS))
     _, want = _oracle_frames(lat, pe, ne, torch.float32)
-    assert frames.shape == want.shape == (1, 3, FRAMES, H, W) and frames.dtype == torch.float32
-    assert (frames - want).abs().max().item() < 2e-5  # two fp32 evaluations of the same graph
+    assert frames.shape == want.shape == (1, 3, FRAMES, H, W) and frames.dtype == str(want.dtype)
+    refgold.assert_close(want, frames, atol=2e-5)  # two fp32 evaluations of the same graph
 
 
 def test_reference_pipeline_call_pins_the_oracle_loop_bf16():
     """In bf16 the loop's rounding points matter (timestep to bf16, CFG combine in bf16, (sigma_next - sigma) rounded to bf16
     by type promotion, fp32 sample): the oracle's loop reproduces the reference pipeline's latents bit for bit."""
     lat, pe, ne = _inputs(6)
-    rt, rv = _reference_modules(bf16)
-    pipe = ref_pipeline.reference_pipeline(rt, rv)
-    seen = {}
-    orig = pipe.decode_latents
-    pipe.decode_latents = lambda z: (seen.setdefault("z", z.clone()), orig(z))[1]
-    frames = ref_pipeline.run(pipe, lat.to(bf16), pe.to(bf16), ne.to(bf16), height=H, width=W, video_length=FRAMES,
-                              num_inference_steps=STEPS)
+
+    def reference_call():
+        pipe = ref_pipeline.reference_pipeline(*_reference_modules(bf16))
+        seen = {}
+        orig = pipe.decode_latents
+        pipe.decode_latents = lambda z: (seen.setdefault("z", z.clone()), orig(z))[1]
+        frames = ref_pipeline.run(pipe, lat.to(bf16), pe.to(bf16), ne.to(bf16), height=H, width=W, video_length=FRAMES,
+                                  num_inference_steps=STEPS)
+        return {"z": seen["z"], "frames": frames}
+
+    ref = refgold.want("ref_pipeline/bf16", reference_call)
     z, want = _oracle_frames(lat, pe, ne, bf16)
-    assert torch.equal(seen["z"], z)
-    assert (frames - want).abs().max().item() < 2e-2
+    refgold.assert_equal(z, ref["z"], rel=3e-2)
+    refgold.assert_close(want, ref["frames"], atol=2e-2, elsewhere_rel=3e-2)
 
 
-def test_reference_pipeline_drives_the_product_modules(monkeypatch):
-    from easyanimate_b200.autoencoder_magvit import AutoencoderKLMagvit
+def test_reference_pipeline_drives_the_product_modules(on_cpu):
+    from easyanimate_b200 import EasyAnimatePipeline
     from easyanimate_b200.transformer3d import EasyAnimateTransformer3DModel
-    cpu_ops.install(monkeypatch)
-    cpu_ops.install_vae(monkeypatch)
-
-    def decode_on_cpu(self, z):  # the product refuses CPU latents (no CPU path); the host logic under test starts behind that guard
-        outs = [self._decode_one(zb) for zb in z.to(bf16)]
-        return outs[0] if len(outs) == 1 else torch.cat(outs, dim=0)
-
-    monkeypatch.setattr(AutoencoderKLMagvit, "_decode", decode_on_cpu)
+    AutoencoderKLMagvit = on_cpu.AutoencoderKLMagvit
     lat, pe, ne = (t.to(bf16) for t in _inputs(7))
     ob = dit.init_weights_(dit.OracleTransformer3D(**CFG), 31).to(bf16)
     ours_t = EasyAnimateTransformer3DModel(**CFG, time_position_encoding_type="3d_rope").to(bf16)
@@ -95,13 +93,13 @@ def test_reference_pipeline_drives_the_product_modules(monkeypatch):
     ours_v = AutoencoderKLMagvit(latent_channels=16, cache_mag_vae=True, spatial_group_norm=True,
                                  mid_block_attention_type="spatial", block_out_channels=list(BOC), scaling_factor=0.7125).to(bf16)
     ours_v.load_state_dict(ov.state_dict(), strict=False)
-    pipe = ref_pipeline.reference_pipeline(ours_t, ours_v)
-    frames = ref_pipeline.run(pipe, lat, pe, ne, height=H, width=W, video_length=FRAMES, num_inference_steps=STEPS)
-    rt, rv = _reference_modules(bf16)
-    want = ref_pipeline.run(ref_pipeline.reference_pipeline(rt, rv), lat, pe, ne, height=H, width=W, video_length=FRAMES,
-                            num_inference_steps=STEPS)
-    assert frames.shape == want.shape == (1, 3, FRAMES, H, W) and frames.dtype == torch.float32
-    rel = ((frames - want).norm() / want.norm()).item()
+    frames = ref_pipeline.run(EasyAnimatePipeline(vae=ours_v, transformer=ours_t), lat, pe, ne, height=H, width=W,
+                              video_length=FRAMES, num_inference_steps=STEPS)
+    want = refgold.want("ref_pipeline/t2v_reference_modules", lambda: ref_pipeline.run(
+        ref_pipeline.reference_pipeline(*_reference_modules(bf16)), lat, pe, ne, height=H, width=W, video_length=FRAMES,
+        num_inference_steps=STEPS))
+    assert tuple(frames.shape) == want.shape == (1, 3, FRAMES, H, W) and frames.dtype == torch.float32
+    rel = refgold.diff(frames, want)[1]
     assert rel < 3e-2, rel  # bf16 round-off of two op orders through 3 CFG steps + decode; a plumbing error is O(1)
 
 
@@ -120,29 +118,30 @@ def _i2v_inputs(seed=9):
     return video, mask, pe, ne
 
 
-def test_reference_inpaint_pipeline_drives_the_product_modules(monkeypatch):
-    """`EasyAnimateInpaintPipeline.__call__` (pipeline_easyanimate_inpaint.py:978-1604), unmodified: VaeImageProcessor ->
-    masked video -> `vae.encode(...)[0].mode()` * scaling_factor -> resize_mask -> inpaint_latents (1 + 16 channels) -> denoise
-    loop with `inpaint_latents=` -> decode_latents.  Once over the reference's transformer + VAE, once over the product's
-    (kernels = torch stand-ins): same start noise (seeded generator), same frames up to bf16 round-off."""
-    import easyanimate_b200.autoencoder_magvit as A
+def test_reference_inpaint_pipeline_drives_the_product_modules(on_cpu):
+    """`EasyAnimateInpaintPipeline.__call__` (pipeline_easyanimate_inpaint.py:978-1604): VaeImageProcessor -> masked video ->
+    `vae.encode(...)[0].mode()` * scaling_factor -> resize_mask -> inpaint_latents (1 + 16 channels) -> denoise loop with
+    `inpaint_latents=` -> decode_latents.  The reference's class over the reference's transformer + VAE (stored), the product's
+    over the product's (kernels = torch stand-ins): same start noise (seeded generator), same frames up to bf16 round-off."""
+    from easyanimate_b200 import EasyAnimateInpaintPipeline
     from easyanimate_b200.transformer3d import EasyAnimateTransformer3DModel
-    from oracle import ref_dit, ref_vae
-    cpu_ops.install(monkeypatch)
-    cpu_ops.install_vae(monkeypatch)
-    monkeypatch.setattr(A, "_require_cuda", lambda t, what: None)  # lift the no-CPU-path guard, nothing else
+    A = on_cpu
     video, mask, pe, ne = _i2v_inputs()
     pe, ne = pe.to(bf16), ne.to(bf16)
     ocfg = {k: v for k, v in I2V_CFG.items() if k in CFG}
     ob = dit.init_weights_(dit.OracleTransformer3D(**ocfg), 51).to(bf16)
     ov = vae.init_weights_(vae.OracleAutoencoderKLMagvit(block_out_channels=list(BOC), with_encoder=True), 52).to(bf16)
 
-    rt = ref_dit.reference_transformer(**I2V_CFG).eval()
-    rt.load_state_dict(ob.state_dict(), strict=True)
-    rv = ref_vae.reference_autoencoder(block_out_channels=BOC).eval()
-    rv.load_state_dict(ov.state_dict(), strict=True)
-    want = ref_pipeline.run_inpaint(ref_pipeline.reference_inpaint_pipeline(rt.to(bf16), rv.to(bf16)), video, mask, pe, ne,
-                                    height=H, width=W, num_inference_steps=STEPS, seed=77)
+    def reference_call():
+        from oracle import ref_dit, ref_vae
+        rt = ref_dit.reference_transformer(**I2V_CFG).eval()
+        rt.load_state_dict(ob.state_dict(), strict=True)
+        rv = ref_vae.reference_autoencoder(block_out_channels=BOC).eval()
+        rv.load_state_dict(ov.state_dict(), strict=True)
+        return ref_pipeline.run_inpaint(ref_pipeline.reference_inpaint_pipeline(rt.to(bf16), rv.to(bf16)), video, mask, pe, ne,
+                                        height=H, width=W, num_inference_steps=STEPS, seed=77)
+
+    want = refgold.want("ref_pipeline/inpaint_reference_modules", reference_call)
 
     ours_t = EasyAnimateTransformer3DModel(**I2V_CFG).to(bf16)
     ours_t.load_state_dict(ob.state_dict(), strict=True)
@@ -153,11 +152,11 @@ def test_reference_inpaint_pipeline_drives_the_product_modules(monkeypatch):
     seen = {}
     enc = ours_v.encode
     ours_v.encode = lambda x, *a, **k: (seen.setdefault("encode_calls", []).append(tuple(x.shape)), enc(x, *a, **k))[1]
-    frames = ref_pipeline.run_inpaint(ref_pipeline.reference_inpaint_pipeline(ours_t, ours_v), video, mask, pe, ne,
+    frames = ref_pipeline.run_inpaint(EasyAnimateInpaintPipeline(vae=ours_v, transformer=ours_t), video, mask, pe, ne,
                                       height=H, width=W, num_inference_steps=STEPS, seed=77)
     assert seen["encode_calls"] == [(1, 3, FRAMES, H, W)]  # the masked video, once (resize_inpaint_mask_directly: no mask encode)
-    assert frames.shape == want.shape == (1, 3, FRAMES, H, W) and frames.dtype == torch.float32
-    rel = ((frames - want).norm() / want.norm()).item()
+    assert tuple(frames.shape) == want.shape == (1, 3, FRAMES, H, W) and frames.dtype == torch.float32
+    rel = refgold.diff(frames, want)[1]
     assert rel < 3e-2, rel
 
 
@@ -166,16 +165,14 @@ CONTROL_CFG = dict(CFG, in_channels=48, time_position_encoding_type="3d_rope", a
 
 
 @pytest.mark.parametrize("with_ref_image", [True, False])
-def test_reference_control_pipeline_drives_the_product_modules(monkeypatch, with_ref_image):
-    """`EasyAnimateControlPipeline.__call__` (pipeline_easyanimate_control.py:833-1282), unmodified: control video ->
-    `vae.encode` -> control_latents (16 channels) + the reference image's latent in frame 0 of 16 more channels
-    (add_ref_latent_in_control_model) -> `transformer(..., control_latents=)` -> decode_latents."""
-    import easyanimate_b200.autoencoder_magvit as A
+def test_reference_control_pipeline_drives_the_product_modules(on_cpu, with_ref_image):
+    """`EasyAnimateControlPipeline.__call__` (pipeline_easyanimate_control.py:833-1282): control video -> `vae.encode` ->
+    control_latents (16 channels) + the reference image's latent in frame 0 of 16 more channels (add_ref_latent_in_control_model)
+    -> `transformer(..., control_latents=)` -> decode_latents.  The reference's class over the reference's modules (stored), the
+    product's over the product's."""
+    from easyanimate_b200 import EasyAnimateControlPipeline
     from easyanimate_b200.transformer3d import EasyAnimateTransformer3DModel
-    from oracle import ref_dit, ref_vae
-    cpu_ops.install(monkeypatch)
-    cpu_ops.install_vae(monkeypatch)
-    monkeypatch.setattr(A, "_require_cuda", lambda t, what: None)
+    A = on_cpu
     g = torch.Generator().manual_seed(13)
     lat = torch.randn(1, 16, LF, H // 8, W // 8, generator=g).to(bf16)
     control = torch.rand(1, 3, FRAMES, H, W, generator=g)
@@ -186,69 +183,24 @@ def test_reference_control_pipeline_drives_the_product_modules(monkeypatch, with
     ov = vae.init_weights_(vae.OracleAutoencoderKLMagvit(block_out_channels=list(BOC), with_encoder=True), 62).to(bf16)
     kw = dict(height=H, width=W, video_length=FRAMES, num_inference_steps=STEPS)
 
-    rt = ref_dit.reference_transformer(**CONTROL_CFG).eval()
-    rt.load_state_dict(ob.state_dict(), strict=True)
-    rv = ref_vae.reference_autoencoder(block_out_channels=BOC).eval()
-    rv.load_state_dict(ov.state_dict(), strict=True)
-    want = ref_pipeline.run_control(ref_pipeline.reference_control_pipeline(rt.to(bf16), rv.to(bf16)), lat, control, ref_image,
-                                    pe, ne, **kw)
+    def reference_call():
+        from oracle import ref_dit, ref_vae
+        rt = ref_dit.reference_transformer(**CONTROL_CFG).eval()
+        rt.load_state_dict(ob.state_dict(), strict=True)
+        rv = ref_vae.reference_autoencoder(block_out_channels=BOC).eval()
+        rv.load_state_dict(ov.state_dict(), strict=True)
+        return ref_pipeline.run_control(ref_pipeline.reference_control_pipeline(rt.to(bf16), rv.to(bf16)), lat, control, ref_image,
+                                        pe, ne, **kw)
+
+    want = refgold.want(f"ref_pipeline/control_reference_modules_{with_ref_image}", reference_call)
     ours_t = EasyAnimateTransformer3DModel(**CONTROL_CFG).to(bf16)
     ours_t.load_state_dict(ob.state_dict(), strict=True)
     ours_v = A.AutoencoderKLMagvit(latent_channels=16, cache_mag_vae=True, spatial_group_norm=True, mid_block_attention_type="spatial",
                                    block_out_channels=list(BOC), scaling_factor=0.7125, mini_batch_encoder=4,
                                    mini_batch_decoder=1).to(bf16)
     ours_v.load_state_dict(ov.state_dict(), strict=True)
-    frames = ref_pipeline.run_control(ref_pipeline.reference_control_pipeline(ours_t, ours_v), lat, control, ref_image, pe, ne, **kw)
-    assert frames.shape == want.shape == (1, 3, FRAMES, H, W) and frames.dtype == torch.float32
-    rel = ((frames - want).norm() / want.norm()).item()
+    frames = ref_pipeline.run_control(EasyAnimateControlPipeline(vae=ours_v, transformer=ours_t), lat, control, ref_image, pe, ne,
+                                      **kw)
+    assert tuple(frames.shape) == want.shape == (1, 3, FRAMES, H, W) and frames.dtype == torch.float32
+    rel = refgold.diff(frames, want)[1]
     assert rel < 3e-2, rel
-
-
-def test_reference_merge_lora_walks_the_product_transformer(monkeypatch):
-    """utils/lora_utils.py:369-431 `merge_lora` (lifted out of the reference file, executed unmodified) resolves
-    `lora_unet__transformer_blocks_0_attn1_to_q`-style keys by attribute walks over `pipeline.transformer` and edits
-    `layer.weight.data`: the product transformer has the same module tree, so the same LoRA file merges into it; after
-    `invalidate_weight_caches()` its forward equals the forward of the reference transformer with the same LoRA merged."""
-    import ast
-    import types
-    from collections import defaultdict
-    from easyanimate_b200.transformer3d import EasyAnimateTransformer3DModel
-    from oracle import ref_dit
-    path = f"{ref_pipeline.REFERENCE_ROOT}/easyanimate/utils/lora_utils.py"
-    fn = [n for n in ast.parse(open(path).read()).body if isinstance(n, ast.FunctionDef) and n.name == "merge_lora"]
-    ns = {"torch": torch, "defaultdict": defaultdict, "load_file": None}
-    exec(compile(ast.Module(body=fn, type_ignores=[]), path, "exec"), ns)
-    cpu_ops.install(monkeypatch)
-    cfg = dict(CFG, time_position_encoding_type="3d_rope")
-    ob = dit.init_weights_(dit.OracleTransformer3D(**CFG), 81).to(bf16)
-    ours = EasyAnimateTransformer3DModel(**cfg).to(bf16)
-    ours.load_state_dict(ob.state_dict(), strict=True)
-    rt = ref_dit.reference_transformer(**cfg).eval().to(bf16)
-    rt.load_state_dict(ob.state_dict(), strict=True)
-    g = torch.Generator().manual_seed(82)
-    lora, d = {}, CFG["num_attention_heads"] * 64
-    for name, (o, i) in {"transformer_blocks_0_attn1_to_q": (d, d), "transformer_blocks_1_attn2_to_v": (d, d),
-                         "transformer_blocks_1_ff_net_2": (d, 4 * d), "transformer_blocks_0_txt_ff_net_0_proj": (4 * d, d)}.items():
-        lora[f"lora_unet__{name}.lora_down.weight"] = torch.randn(4, i, generator=g) * 0.1
-        lora[f"lora_unet__{name}.lora_up.weight"] = torch.randn(o, 4, generator=g) * 0.1
-        lora[f"lora_unet__{name}.alpha"] = torch.tensor(2.0)
-    lat = torch.randn(1, 16, LF, H // 8, W // 8, generator=g).to(bf16)
-    enc = (torch.randn(1, 9, 128, generator=g) * 3).to(bf16)
-    t = torch.tensor([700.0]).to(bf16)
-    rope = dit.rope_for_video(H, W, LF)
-
-    def run(m):
-        with torch.no_grad():
-            return m(lat, t, encoder_hidden_states=enc, image_rotary_emb=rope, return_dict=False)[0]
-
-    before = run(ours)
-    for m in (ours, rt):
-        ns["merge_lora"](types.SimpleNamespace(transformer=m, text_encoder=None), None, 0.8, state_dict=dict(lora), transformer_only=True)
-    ours.invalidate_weight_caches()
-    after, want = run(ours), run(rt)
-    theirs = rt.state_dict()
-    for k, a in ours.state_dict().items():
-        assert torch.equal(a, theirs[k]), k  # the same edits landed in the same parameters
-    assert not torch.equal(theirs["transformer_blocks.0.attn1.to_q.weight"], ob.state_dict()["transformer_blocks.0.attn1.to_q.weight"])
-    rel = ((after.float() - want.float()).norm() / want.float().norm()).item()
-    assert rel < 2e-2 and not torch.equal(after, before), rel
